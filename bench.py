@@ -134,11 +134,31 @@ def synthetic_clips(B, T, seed):
     return x.pin_memory() if torch.cuda.is_available() else x
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, rank=0, world=1):
+    """`--dump-outputs`: write what the timed path returned in its last step as out_dir/<name>.npy in float32 (with
+    several ranks, out_dir/<name>_rank<r>.npy per rank), so that two builds run with the same arguments can be compared
+    output for output.  An array that does not fit the 64 MB left for all files is cut to a fixed, seeded sample of its
+    rows (first dimension: the batch of sequences), the same rows on every run."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES // world
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > budget and a.ndim > 0:
+            keep = max(1, budget // (a.nbytes // a.shape[0]))
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        budget -= a.nbytes
+        np.save(os.path.join(out_dir, name + (f"_rank{rank}" if world > 1 else "") + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------ CPU reference arm
-def cpu_reference_rate(model, T, budget_s=20.0, batch=2, max_iters=12):
+def cpu_reference_rate(model, T, budget_s=20.0, batch=2, max_iters=12, warmup=1):
     """The reference's own CPU forward, restated op-for-op with torch CPU ops (oracle/dstformer_torch_cpu.py; the
     reference itself is PyTorch-only Python and cannot travel to the GPU box).  Uses the host thread count that a
-    short calibration finds fastest (torch's default = all cores is pathological on 100+-thread hosts)."""
+    short calibration finds fastest (torch's default = all cores is pathological on 100+-thread hosts).  Times
+    max_iters forwards, fewer once budget_s seconds have passed (budget_s=None: exactly max_iters)."""
     from oracle import dstformer_oracle as O
     from oracle import dstformer_torch_cpu as OT
     cfg = O.BASE if model == "base" else O.LITE
@@ -156,10 +176,11 @@ def cpu_reference_rate(model, T, budget_s=20.0, batch=2, max_iters=12):
             best_t, best_n = dt, n
     torch.set_num_threads(best_n)
     x = torch.from_numpy(O.make_input(batch, T, cfg.num_joints, 1))
-    OT.forward(P, x, cfg.depth, cfg.num_heads, cfg.eps)           # warm-up
+    for _ in range(warmup):
+        OT.forward(P, x, cfg.depth, cfg.num_heads, cfg.eps)
     times = []
     t_start = time.perf_counter()
-    while len(times) < max_iters and (not times or (time.perf_counter() - t_start) < budget_s):
+    while len(times) < max_iters and (budget_s is None or not times or (time.perf_counter() - t_start) < budget_s):
         t0 = time.perf_counter()
         OT.forward(P, x, cfg.depth, cfg.num_heads, cfg.eps)
         times.append(time.perf_counter() - t0)
@@ -173,8 +194,8 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, args.steps)
-    cb = cpu_reference_rate(args.model, args.frames, budget_s=min(120.0, 8.0 * steps), batch=2, max_iters=steps + args.warmup)
+    steps = args.steps
+    cb = cpu_reference_rate(args.model, args.frames, budget_s=None, batch=2, max_iters=steps, warmup=args.warmup)
     line = {
         "impl": "reference", "metric": f"sequences/sec DSTformer-{args.model} fwd (Bx{args.frames}x17)",
         "value": cb["value"], "unit": "sequences/sec", "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup,
@@ -195,11 +216,12 @@ def _barrier(dist, device):
 
 
 def train_record(args, device, world, rank, local_rank, dist, D, model_name="base", batch=128, frames=243, math="bf16",
-                 steps=20, warmup=3, e2e_steps=0):
+                 steps=20, warmup=3, e2e_steps=0, dump_dir=None):
     """SURVEY.md 8d config 3 (N=1) / config 4 (N>1): one pretrain step = forward (saved residual stream) -> fused pretrain
     loss (mpjpe + 0.5 n_mpjpe + 20 velocity, train.py:178-191) -> native backward -> gradient all-reduce over the ranks
     (N>1, per depth, overlapped with the backward) -> fused AdamW -> weight re-pack at the next forward.
-    Returns the record (identical on every rank: times are max over ranks)."""
+    Returns the record (identical on every rank: times are max over ranks).  dump_dir: see dump_outputs; the last timed
+    step's loss parts, predicted poses and a fixed strided sample of 1M updated parameters."""
     from motionbert_b200 import _lib
     from motionbert_b200.loss import pretrain_loss_3d
     model = build_model(model_name, device, math).train()
@@ -218,10 +240,10 @@ def train_record(args, device, world, rank, local_rank, dist, D, model_name="bas
     def step(x, gt):
         opt.zero_grad(set_to_none=True)
         pred = model(x)
-        loss, _parts = pretrain_loss_3d(pred, gt, 0.5, 20.0)
+        loss, parts = pretrain_loss_3d(pred, gt, 0.5, 20.0)
         loss.backward()       # world > 1: gradients are averaged over the ranks inside the backward (phase by phase)
         opt.step()
-        return loss
+        return loss, parts, pred
 
     for _ in range(warmup):
         step(x_dev, gt_dev)
@@ -232,13 +254,18 @@ def train_record(args, device, world, rank, local_rank, dist, D, model_name="bas
     _barrier(dist, device)
     ev0.record()
     for _ in range(steps):
-        loss = step(x_dev, gt_dev)
+        loss, parts, pred = step(x_dev, gt_dev)
     ev1.record()
     _barrier(dist, device)
     ms_per_step = D.max_over_ranks(ev0.elapsed_time(ev1), device) / steps
     sampler.stop_flag = True
     sampler.join(timeout=3)
     clocks = sampler.summary()
+    if dump_dir is not None:
+        flat = torch.cat([p.detach().reshape(-1) for p in params])
+        dump_outputs(dump_dir, {"loss_parts": parts, "params_sample": flat[::max(1, flat.numel() >> 20)][:1 << 20],
+                                "pred": pred}, rank, world)
+        del flat
     last = float(loss.detach())
     e2e = None
     if e2e_steps > 0:
@@ -247,7 +274,7 @@ def train_record(args, device, world, rank, local_rank, dist, D, model_name="bas
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(e2e_steps):
-            last = float(step(x_host.to(device, non_blocking=True), gt_host.to(device, non_blocking=True)).item())
+            last = float(step(x_host.to(device, non_blocking=True), gt_host.to(device, non_blocking=True))[0].item())
         e1.record()
         _barrier(dist, device)
         e2e_ms = D.max_over_ranks(e0.elapsed_time(e1), device) / e2e_steps
@@ -284,7 +311,7 @@ def train_record(args, device, world, rank, local_rank, dist, D, model_name="bas
 def run_train(args, device, world, rank, local_rank, dist, D):
     """`--mode train`: the training step as the headline line (supplementary to the forward line)."""
     rec = train_record(args, device, world, rank, local_rank, dist, D, args.model, args.batch, args.frames, args.math,
-                       steps=args.steps, warmup=args.warmup, e2e_steps=args.steps)
+                       steps=args.steps, warmup=args.warmup, e2e_steps=args.steps, dump_dir=args.dump_outputs)
     peaks = load_peaks()
     line = {
         "metric": rec["metric"], "value": rec["value"], "unit": "sequences/sec", "n_gpus": world, "steps": args.steps,
@@ -454,7 +481,14 @@ def main():
     ap.add_argument("--kernel-flags", type=lambda v: int(v, 0), default=0, help="MB_FLAG_* bits for A/B runs (e.g. 0x40 = BF16x3 attention inside F16C)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline forward only (skip train / lite sweep / eager sub-records)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32, "
+                         "64 MB at most): forward: pose_3d (B, T, 17, 3); train: pred, loss_parts, params_sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs records the native path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.batch is None:
         args.batch = 128 if args.mode == "train" else 256
@@ -508,6 +542,8 @@ def main():
     sampler.join(timeout=3)
     clocks = sampler.summary()
     value = world * B / (ms_per_step * 1e-3)
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, {"pose_3d": out}, rank, world)
 
     # ---- the output that was timed, against the CPU oracle (rank 0; a miss fails the run)
     parity = None
@@ -641,7 +677,7 @@ def main():
             lite._kernel_flags = args.kernel_flags
             for t_len in (27, 81, 243):
                 xl = synthetic_clips(512, t_len, seed=7 + rank).to(device)
-                ms, _o = forward_rate(lite, xl, max(5, min(args.steps, 10)), 3, dist, device, D)
+                ms, _o = forward_rate(lite, xl, args.steps, 3, dist, device, D)
                 fl = flops_per_sequence(256, 1024, t_len) * 512
                 sweep.append({"T": t_len, "B_per_gpu": 512, "value": world * 512 / (ms * 1e-3), "unit": "sequences/sec",
                               "ms_per_step": ms, "whole_step_tflops": fl / (ms * 1e-3) / 1e12,
@@ -652,14 +688,16 @@ def main():
         guarded("lite_sweep", lite_sweep)
         # ---- config 3 (N = 1) / config 4 (N > 1): the pretrain step
         guarded("train", lambda: train_record(args, device, world, rank, local_rank, dist, D, "base", 128, 243, "bf16",
-                                              steps=20, warmup=3))
+                                              steps=args.steps, warmup=3))
         # ---- the reference's forward in torch eager on this same GPU (N = 1 only: a per-GPU comparator)
         if world == 1:
             guarded("gpu_eager_baseline",
-                    lambda: gpu_eager_baseline(build_model(args.model, device, args.math), args.model, T, device))
+                    lambda: gpu_eager_baseline(build_model(args.model, device, args.math), args.model, T, device,
+                                               iters=args.steps))
             # ... and its training step (config 3's comparator: autocast-bf16 / TF32 eager fwd + autograd bwd + AdamW)
             guarded("gpu_eager_train_baseline",
-                    lambda: gpu_eager_train_baseline(build_model(args.model, device, args.math), args.model, T, device))
+                    lambda: gpu_eager_train_baseline(build_model(args.model, device, args.math), args.model, T, device,
+                                                     iters=args.steps))
 
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_reference_rate(args.model, T, budget_s=20.0)

@@ -1,4 +1,5 @@
-"""bench.py's host-side pieces that can run without a GPU: the FLOP bookkeeping behind `roofline`, and the torch-eager
+"""bench.py's host-side pieces that can run without a GPU: the FLOP bookkeeping behind `roofline`, the output dump of
+`--dump-outputs`, and the torch-eager
 training comparator (SURVEY.md 8d config 3) exercised on the CPU at a toy size (on the GPU box it runs on cuda:0)."""
 import os
 import sys
@@ -19,6 +20,25 @@ def test_flop_bookkeeping_matches_the_survey_numbers():
     for t, g in ((243, 142.093), (81, 45.080), (27, 14.773)):
         assert abs(bench.flops_per_sequence(256, 1024, t) / 1e9 - g) < 0.01
     assert bench.gemm_flops_per_sequence(512, 1024, 243) < bench.flops_per_sequence(512, 1024, 243)
+
+
+def test_dump_outputs_writes_float32_within_the_size_cap_and_samples_the_same_rows(monkeypatch, tmp_path):
+    import numpy as np
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 16)
+    big = torch.arange(1000 * 32, dtype=torch.float64).reshape(1000, 32)
+    arrays = {"loss_parts": torch.tensor([1.0, 2.0, 3.0, 6.0]), "pose_3d": big}
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    a = {f.stem: np.load(f) for f in (tmp_path / "a").iterdir()}
+    b = {f.stem: np.load(f) for f in (tmp_path / "b").iterdir()}
+    assert sorted(a) == ["loss_parts", "pose_3d"] and all(v.dtype == np.float32 for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 1 << 16
+    assert np.array_equal(a["loss_parts"], [1, 2, 3, 6])
+    rows = a["pose_3d"][:, 0] / 32                                   # whole rows of the batch, in order
+    assert 0 < len(rows) < 1000 and np.all(np.diff(rows) > 0) and np.array_equal(a["pose_3d"], big.float().numpy()[rows.astype(int)])
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    bench.dump_outputs(str(tmp_path / "r"), {"pose_3d": big[:10]}, rank=1, world=2)
+    assert [f.name for f in (tmp_path / "r").iterdir()] == ["pose_3d_rank1.npy"]
 
 
 def test_eager_training_comparator_runs_a_real_optimizer_step(monkeypatch):

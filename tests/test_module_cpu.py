@@ -1,6 +1,7 @@
 """Drop-in boundary checks that need no GPU: parameter tree, init known-answers, state_dict round trip,
 shim import path, loud failure on CPU tensors (SURVEY.md section 8 rows a1, a13, a14, b)."""
 import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -9,7 +10,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT, build_module, manifest
+from conftest import GOLD, ROOT, build_module, manifest
 from oracle import dstformer_oracle as O
 
 
@@ -78,21 +79,70 @@ def test_cpu_tensor_fails_loudly_no_fallback():
         m(torch.zeros(1, 4, 16, 3))
 
 
-def test_shim_shadows_exactly_the_reference_module():
-    """lib/ is a namespace package in the reference: shim first on sys.path replaces only lib.model.DSTformer."""
+# lib/utils/learning.py of the stand-in checkout: constructs the backbone with recorded constructor arguments
+_STANDIN_FACTORY = '''
+import importlib
+from functools import partial
+
+from lib.model.DSTformer import DSTformer
+
+
+def _arg(v):
+    if isinstance(v, dict) and "partial" in v:
+        mod, _, name = v["partial"].rpartition(".")
+        return partial(getattr(importlib.import_module(mod), name), *v["args"], **v["keywords"])
+    return v
+
+
+def load_backbone(recorded_kwargs):
+    return DSTformer(**{k: _arg(v) for k, v in recorded_kwargs.items()})
+'''
+
+_SHIM_CHECK = '''
+import json, sys
+import motionbert_b200
+import lib.model.drop as dr
+from lib.utils.learning import load_backbone
+from oracle import dstformer_oracle as O
+gold = json.load(open(sys.argv[1]))
+for name, c in gold["configs"].items():
+    m = load_backbone(c["kwargs"])
+    assert type(m) is motionbert_b200.DSTformer, name
+    assert m.eps == c["kwargs"]["norm_layer"]["keywords"]["eps"] == 1e-6, name
+    shapes = {k: tuple(v.shape) for k, v in m.state_dict().items()}
+    assert shapes == O.param_shapes({"base": O.BASE, "lite": O.LITE}[name]), name
+assert dr.__file__.startswith(sys.argv[2]), dr.__file__
+print("ok")
+'''
+
+
+def test_shim_shadows_exactly_the_reference_module(tmp_path):
+    """lib/ is a namespace package in the reference: shim first on sys.path replaces only lib.model.DSTformer.
+
+    The reference's side is a stand-in checkout laid out as tests/golden/load_backbone.json records the real one
+    (oracle/make_golden_backbone.py): the same namespace packages and lib/model modules, a DSTformer module that must
+    never be imported, and a factory passing the constructor arguments the reference's load_backbone was recorded
+    passing for DSTformer-base and -Lite."""
     code = ("import lib.model.DSTformer as D, motionbert_b200; "
             "assert D.DSTformer is motionbert_b200.DSTformer; print('ok')")
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "shim"), ROOT]))
     r = subprocess.run([sys.executable, "-P", "-c", code], capture_output=True, text=True, env=env)
     assert r.returncode == 0 and "ok" in r.stdout, r.stderr
-    if os.path.isdir("/root/reference/lib"):
-        code = ("from types import SimpleNamespace as NS; from lib.utils.learning import load_backbone; import motionbert_b200;"
-                "m = load_backbone(NS(backbone='DSTformer', dim_feat=256, dim_rep=512, depth=5, num_heads=8, mlp_ratio=4,"
-                " maxlen=243, num_joints=17)); assert type(m) is motionbert_b200.DSTformer; assert m.eps == 1e-6;"
-                "import lib.model.drop as dr; assert 'reference' in dr.__file__; print('ok')")
-        env["PYTHONPATH"] += os.pathsep + "/root/reference"
-        r = subprocess.run([sys.executable, "-P", "-c", code], capture_output=True, text=True, env=env)
-        assert r.returncode == 0 and "ok" in r.stdout, r.stderr
+    gold_path = os.path.join(GOLD, "load_backbone.json")
+    with open(gold_path) as f:
+        gold = json.load(f)
+    assert gold["namespace_packages"] == ["lib", "lib.model", "lib.utils"]
+    ref = tmp_path / "MotionBERT"
+    for pkg in gold["namespace_packages"]:
+        (ref / pkg.replace(".", os.sep)).mkdir(parents=True, exist_ok=True)
+    for mod in gold["lib_model_modules"]:
+        (ref / "lib" / "model" / f"{mod}.py").write_text("")
+    (ref / "lib" / "model" / "DSTformer.py").write_text("raise ImportError('the shim did not shadow lib.model.DSTformer')\n")
+    (ref / "lib" / "utils" / "learning.py").write_text(_STANDIN_FACTORY)
+    env["PYTHONPATH"] += os.pathsep + str(ref)
+    r = subprocess.run([sys.executable, "-P", "-c", _SHIM_CHECK, gold_path, str(ref)], capture_output=True, text=True,
+                       env=env)
+    assert r.returncode == 0 and "ok" in r.stdout, r.stderr
 
 
 def test_backward_phase_of_every_parameter_matches_its_name():
